@@ -13,6 +13,13 @@ histograms.  `value` is whole-job entries/s (CUDA events, max over ranks); `e2e`
 host-buffer C-ABI call (pinned host memory in, host results out, copies inside the timed region, the same exact
 multi-GPU path at N>1).  `secondary` holds BASELINE configs[2..4] as written (streamed chunks, persistent tables,
 duplicates straddling chunks and GPUs).  Prints ONE JSON line on rank 0.
+
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+also writes what the timed path returned in its last step to DIR/<name>.npy (rank 0's shard): the per-entry outputs of
+a fixed, seeded sample of entries (`entry_index`; all entries when there are at most DUMP_ENTRIES) and the whole
+per-issuer / per-status histograms.  The corpus is seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -33,6 +40,8 @@ NOW_SEC = 1767225600
 NOW_NS = NOW_SEC * 10**9
 SEED = 20260922
 README_FILTER = b"Let's Encrypt, ISRG"
+# entries sampled by --dump-outputs: 32 fingerprint bytes as float32 + 5 scalars each, about 20 MB in all
+DUMP_ENTRIES = 1 << 17
 
 WORKLOADS = {
     # BASELINE.json configs[1]: SHA-256 fingerprint + KnownCertificates dedup (no CN filter, expired kept)
@@ -74,7 +83,12 @@ def parse_args():
     ap.add_argument("--no-secondary", action="store_true", help="skip the BASELINE configs[2..4] streaming runs")
     ap.add_argument("--secondary-entries", type=int, default=0, help="entries per GPU of each streaming run (default: as written)")
     ap.add_argument("--cpu-sample", type=int, default=0, help="entries in the CPU sample (default: auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the last timed step's outputs (seeded sample of entries + histograms) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------- clocks
@@ -162,7 +176,8 @@ def host_threads():
 
 def go_probe():
     """BASELINE.md §3 Variant A / SURVEY §8(c): use the Go engine when the box has a Go toolchain AND the reference's
-    module dependencies are resolvable offline.  Returns (usable, one-line description)."""
+    module dependencies are resolvable offline (reference checkout: $CTMR_REFERENCE_DIR).  Returns (usable, one-line
+    description)."""
     go = shutil.which("go")
     if not go:
         return False, "`go version`: command not found on this box"
@@ -170,9 +185,9 @@ def go_probe():
         ver = subprocess.run([go, "version"], capture_output=True, text=True, timeout=20).stdout.strip()
     except Exception as e:  # noqa: BLE001
         return False, f"`go version` failed: {e}"
-    ref = "/root/reference"
+    ref = os.environ.get("CTMR_REFERENCE_DIR", "")
     if not os.path.isdir(ref):
-        return False, f"{ver}; the reference sources (/root/reference) are not on this box"
+        return False, f"{ver}; no reference checkout (set CTMR_REFERENCE_DIR to one)"
     env = dict(os.environ, GOFLAGS="-mod=mod", GOPROXY="off")
     r = subprocess.run([go, "list", "./storage"], cwd=ref, capture_output=True, text=True, env=env, timeout=120)
     if r.returncode != 0:
@@ -381,6 +396,20 @@ def main():
     map_ms = allmax(db.profile_last()[0])   # K_map's CUDA-event duration (sum over the step's 4 launches) in the LAST timed step
     db.check_device(stream.cuda_stream)
     counts, stat = hist[: cfg.n_issuers].clone(), hist[cfg.n_issuers:].clone()
+    if args.dump_outputs and rank == 0:
+        pick = np.sort(np.random.default_rng(SEED).choice(n, min(n, DUMP_ENTRIES), replace=False))
+        sel = torch.from_numpy(pick).to(dev)
+        dump = {"entry_index": pick.astype(np.float64), "status": status[sel].cpu().numpy().astype(np.float32),
+                "exp_hour": exp_hour[sel].cpu().numpy().astype(np.float64),
+                "was_unknown": was_unknown[sel].cpu().numpy().astype(np.float32),
+                "first_issuer_hour": first[sel].cpu().numpy().astype(np.float32),
+                "issuer_counts": counts.cpu().numpy().astype(np.float64), "status_counters": stat.cpu().numpy().astype(np.float64)}
+        if not args.no_fingerprint:
+            dump["sha256"] = sha[sel].cpu().numpy().astype(np.float32)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+        del sel
 
     # ---- the timed result is the real thing: size-independent checks on the LAST timed step's outputs ----------
     truth_id = torch.empty(n, dtype=torch.int64, device=dev)
