@@ -15,7 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libctmr.so")
-SOURCES = ["ctmr_map.cu", "ctmr_reduce.cu", "ctmr_api.cu", "ctmr_pipeline.cu", "ctmr_frontend.cu", "ctmr_frontend_api.cu", "ctmr_synth_kernels.cu", "ctmr_synth_pages.cu"]
+SOURCES = ["ctmr_map.cu", "ctmr_reduce.cu", "ctmr_api.cu", "ctmr_pipeline.cu", "ctmr_frontend.cu", "ctmr_frontend_api.cu", "ctmr_sets.cu", "ctmr_synth_kernels.cu", "ctmr_synth_pages.cu"]
 # measured-and-rejected K_map variants (v1 global-memory walk, dynamic scheduling, TMA bulk loader): only with CTMR_EXPERIMENTS=1
 EXPERIMENT_SOURCES = ["ctmr_map_alt.cu"]
 DEPS = SOURCES + EXPERIMENT_SOURCES + ["ctmr_ctx.cuh", "ctmr_kernels.cuh", "ctmr_common.cuh", "ctmr_stream.cuh", "ctmr_device.cuh", "ctmr_synth.h",

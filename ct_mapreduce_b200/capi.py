@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(HERE, "libctmr.so")
 ST_OK, ST_PARSE_ERR, ST_FILTER_CA, ST_FILTER_EXPIRED, ST_FILTER_CN, ST_NO_ISSUER, ST_ISSUER_PARSE_ERR, ST_SERIAL_TOO_LONG = range(8)
 ST_COUNT = 8
 ISSUER_NONE = 0xFFFFFFFF
+MAX_SERIAL = 39
 ISSUER_BAD = 0xFFFFFFFE
 F_NO_FINGERPRINT = 1
 E_INVALID = -1
@@ -40,6 +41,9 @@ EXPORTS = [
     "ctmr_group_snapshot_size", "ctmr_group_snapshot_save", "ctmr_group_snapshot_load",
     "ctmr_peer_export", "ctmr_peer_attach", "ctmr_peer_barrier_device", "ctmr_peer_allreduce_histogram_device",
     "ctmr_bind_host_to_device", "ctmr_peer_rounds", "ctmr_peer_round_entries",
+    # the sets read back: list, members, canonical export / import
+    "ctmr_list_sets", "ctmr_set_members", "ctmr_export_sets", "ctmr_import_sets",
+    "ctmr_group_list_sets", "ctmr_group_set_members", "ctmr_group_export_sets", "ctmr_group_import_sets",
 ]
 PEER_HANDLE_BYTES = 256
 PEER_ROUNDS = 8   # default; peer_rounds() asks the library (environment override)
@@ -100,6 +104,22 @@ class SynthCfg(C.Structure):
         ("len_lo", C.c_uint32), ("len_hi", C.c_uint32), ("dup_mode", C.c_uint32), ("reserved", C.c_uint32),
         ("now_sec", C.c_int64),
     ]
+
+
+class SetInfo(C.Structure):
+    """ctmr_set_info (include/ctmr.h)."""
+    _fields_ = [("issuer_digest", C.c_uint8 * 32), ("exp_hour", C.c_int64), ("count", C.c_uint64), ("member_off", C.c_uint64)]
+
+
+SET_INFO_DTYPE = np.dtype([("issuer_digest", "u1", (32,)), ("exp_hour", "<i8"), ("count", "<u8"), ("member_off", "<u8")])
+assert SET_INFO_DTYPE.itemsize == 56
+
+
+class SetExport(C.Structure):
+    """ctmr_set_export (include/ctmr.h)."""
+    _fields_ = [("next_index", C.c_uint64), ("n_sets", C.c_uint64), ("n_members", C.c_uint64), ("serial_bytes", C.c_uint64),
+                ("sets", C.c_void_p), ("sets_cap", C.c_uint64), ("serials", C.c_void_p), ("serials_cap", C.c_uint64),
+                ("serial_off", C.c_void_p), ("first_index", C.c_void_p), ("members_cap", C.c_uint64)]
 
 
 KEY_BYTES = 64
@@ -196,6 +216,11 @@ def load():
     L.ctmr_peer_rounds.restype = u32
     L.ctmr_peer_round_entries.argtypes = [u64]
     L.ctmr_peer_round_entries.restype = u64
+    for pre in ("ctmr_", "ctmr_group_"):
+        getattr(L, pre + "list_sets").argtypes = [vp, i64, i64, vp, u64, C.POINTER(u64)]
+        getattr(L, pre + "set_members").argtypes = [vp, i64, vp, vp, u64, vp, vp, u64, C.POINTER(u64)]
+        getattr(L, pre + "export_sets").argtypes = [vp, C.POINTER(SetExport)]
+        getattr(L, pre + "import_sets").argtypes = [vp, C.POINTER(SetExport)]
     for name in EXPORTS:
         getattr(L, name)  # every symbol include/ctmr.h declares must resolve
     _lib = L

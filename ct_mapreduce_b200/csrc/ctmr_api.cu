@@ -1040,12 +1040,23 @@ int preload_impl(ctmr_ctx* c, int64_t exp_hour, const uint8_t digest[32], const 
         std::memcpy(keys[i].serial, serial_blob + serial_offsets[i], len);
         keys[i].valid = 1;
     }
-    rc = ensure_scratch(c, n);
+    return reduce_keys_host(c, keys.data(), n);
+}
+
+int reduce_keys_host(ctmr_ctx* c, const ctmr_key* keys, uint64_t n) {
+    CU(c, cudaSetDevice(c->device));
+    // in chunks of the scratch size: a preload's chunks come in index order, an import's keys are distinct, so
+    // lowest-index-wins holds across the chunks either way
+    constexpr uint64_t kChunk = 1ull << 20;
+    int rc = ensure_scratch(c, std::min(n, kChunk));
     if (rc) return rc;
-    CU(c, cudaMemcpyAsync(c->keys_scratch, keys.data(), n * sizeof(ctmr_key), cudaMemcpyHostToDevice, c->stream));
-    rc = reduce_on(c, c->keys_scratch, n, c->slot_scratch, c->pair_scratch, c->bits_scratch, c->bits_scratch + n, c->stream);
-    if (rc) return rc;
-    CU(c, cudaStreamSynchronize(c->stream));
+    for (uint64_t lo = 0; lo < n; lo += c->scratch_cap) {
+        const uint64_t m = std::min(n - lo, c->scratch_cap);
+        CU(c, cudaMemcpyAsync(c->keys_scratch, keys + lo, m * sizeof(ctmr_key), cudaMemcpyHostToDevice, c->stream));
+        rc = reduce_on(c, c->keys_scratch, m, c->slot_scratch, c->pair_scratch, c->bits_scratch, c->bits_scratch + m, c->stream);
+        if (rc) return rc;
+        CU(c, cudaStreamSynchronize(c->stream));
+    }
     return ctmr_check_device(c, nullptr);
 }
 }  // namespace ctmr_host

@@ -10,6 +10,7 @@
 #include <mutex>
 #include <new>
 #include <string>
+#include <thread>
 #include <unordered_map>
 #include <vector>
 
@@ -256,5 +257,28 @@ void stages_destroy(ctmr_ctx* c);
 int pem_ensure(ctmr_ctx* c, PemStage& ps, uint64_t entries, uint64_t der_bytes);
 int pem_chunk(ctmr_ctx* c, PemStage& ps, const uint8_t* blob, const uint64_t* offsets, const uint32_t* lens, const uint8_t* select,
               uint64_t cnt, const ctmr_out* out, uint64_t first, uint64_t* base, cudaStream_t s);
+// host-built key records through the reduce path of c (insert, resolve, pairs), synchronous; every key must be one c owns
+int reduce_keys_host(ctmr_ctx* c, const ctmr_key* keys, uint64_t n);
+
+// a member's error becomes the group's
+inline int group_fail(ctmr_group* g, ctmr_ctx* c, int rc) {
+    if (g && c) g->err = c->err;
+    return rc;
+}
+
+// fn(r) for every member, on one thread each (the members' calls wait on the host: issuer round trips, D2H); sequential if
+// threads cannot be had.  No exception leaves this function (C ABI).
+template <class F>
+void for_each_member(uint32_t W, std::vector<int>& rcs, F fn) {
+    rcs.assign(W, CTMR_OK);
+    std::vector<std::thread> th;
+    uint32_t started = 0;
+    try {
+        for (; started < W; ++started) th.emplace_back([&rcs, &fn, r = started] { rcs[r] = fn(r); });
+    } catch (...) {
+    }
+    for (std::thread& t : th) t.join();
+    for (uint32_t r = started; r < W; ++r) rcs[r] = fn(r);
+}
 
 }  // namespace ctmr_host

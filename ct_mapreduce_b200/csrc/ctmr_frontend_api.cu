@@ -303,21 +303,6 @@ int process_raw_single(ctmr_ctx* c, const ctmr_raw_batch* b, ctmr_raw_out* out) 
     return ctmr_check_device(c, nullptr);
 }
 
-// fn(r) for every member, on one thread each (the halves of a chunk wait on the host: issuer round trips, D2H); sequential if
-// threads cannot be had.  No exception leaves this function (C ABI).
-template <class F>
-void for_each_member(uint32_t W, std::vector<int>& rcs, F fn) {
-    rcs.assign(W, CTMR_OK);
-    std::vector<std::thread> th;
-    uint32_t started = 0;
-    try {
-        for (; started < W; ++started) th.emplace_back([&rcs, &fn, r = started] { rcs[r] = fn(r); });
-    } catch (...) {
-    }
-    for (std::thread& t : th) t.join();
-    for (uint32_t r = started; r < W; ++r) rcs[r] = fn(r);
-}
-
 // One round of the path over the members' device-resident chunks: map + route, [events], owner passes, [events], pull,
 // [string identities: insert, events, read-back].  Each member works on its own stream; rounds are serialised by the
 // callers' fe_back, which is also what orders the rounds for lowest-index-wins.

@@ -137,10 +137,6 @@ struct Slice {
     uint64_t first_index = 0;     // global index of entry lo
 };
 
-int group_fail(ctmr_group* g, ctmr_ctx* c, int rc) {
-    if (g && c) g->err = c->err;
-    return rc;
-}
 
 // rounds x members.  Every slice respects the entry budget and the byte budget of a stage.
 int plan_rounds(ctmr_ctx* c0, uint32_t W, const BatchArgs& a, std::vector<std::vector<Slice>>& plan) {

@@ -10,6 +10,11 @@ points, and exposes the results under the reference's names:
                                        <- KnownCertificates.Count (storage/knowncertificates.go:57-63)
     GpuCertDatabase.issuer_counts      <- the per-issuer sum of cmd/storage-statistics/storage-statistics.go:44-53
     GpuCertDatabase.status_counters    <- metrics certIsFilteredOut.{CA,expired,cn-filtered}, insertCTWorker.Inserted
+    GpuCertDatabase.list_sets          <- GetIssuerAndDatesFromCache + Count() (storage/filesystemdatabase.go:59-100)
+    GpuCertDatabase.get_known_certificates(exp_hour, issuer).known()
+                                       <- KnownCertificates.Known (storage/knowncertificates.go:65-96)
+    GpuCertDatabase.export_sets / import_sets
+                                       <- the Redis state in canonical form, portable across table sizes and group sizes
 
 All arithmetic happens in the CUDA kernels; nothing here parses, hashes or de-duplicates.
 """
@@ -61,6 +66,62 @@ class KnownCertificatesView:
         self._db._check(self._db._lib.ctmr_set_cardinality(self._db._h, self.exp_hour, d, C.byref(out)))
         return out.value
 
+    def known(self) -> list:
+        """The set's serials (raw octets), in first-seen order (KnownCertificates.Known, knowncertificates.go:65-96)."""
+        return self._db.set_members(self.exp_hour, self.issuer_digest)[0]
+
+
+@dataclass
+class SetExport:
+    """Canonical export of the known-certificate sets (include/ctmr.h, "the sets read back"): sets by (issuer digest,
+    exp_hour), members of a set by first index.  Member k of set j: serials[serial_off[k]:serial_off[k+1]], first_index[k],
+    for k in [sets[j]["member_off"], sets[j]["member_off"] + sets[j]["count"])."""
+    next_index: int
+    sets: np.ndarray         # capi.SET_INFO_DTYPE [n_sets]
+    serials: np.ndarray      # uint8 [serial_bytes]
+    serial_off: np.ndarray   # uint64 [n_members + 1]
+    first_index: np.ndarray  # uint64 [n_members]
+
+    @property
+    def n_members(self) -> int:
+        return int(self.first_index.size)
+
+    def members(self, j: int):
+        """[(serial bytes, first index)] of set j."""
+        lo = int(self.sets[j]["member_off"])
+        return [(self.serials[int(self.serial_off[k]):int(self.serial_off[k + 1])].tobytes(), int(self.first_index[k]))
+                for k in range(lo, lo + int(self.sets[j]["count"]))]
+
+    def tobytes(self) -> bytes:
+        """Every array back to back: equal exports are equal byte strings."""
+        return b"".join([np.uint64(self.next_index).tobytes(), self.sets.tobytes(), self.serials.tobytes(),
+                         np.ascontiguousarray(self.serial_off, np.uint64).tobytes(),
+                         np.ascontiguousarray(self.first_index, np.uint64).tobytes()])
+
+    def __eq__(self, other) -> bool:
+        return isinstance(other, SetExport) and self.tobytes() == other.tobytes()
+
+    @staticmethod
+    def merge(parts) -> "SetExport":
+        """The exports of the shards of one group (disjoint sets) -> the group's export, canonical order."""
+        parts = list(parts)
+        order = sorted((bytes(p.sets[j]["issuer_digest"]), int(p.sets[j]["exp_hour"]), i, j)
+                       for i, p in enumerate(parts) for j in range(p.sets.size))
+        sets = np.zeros(len(order), capi.SET_INFO_DTYPE)
+        serials, first, lens, run = [], [], [], 0
+        for out_j, (_, _, i, j) in enumerate(order):
+            sets[out_j] = parts[i].sets[j]
+            sets[out_j]["member_off"] = run
+            for ser, fi in parts[i].members(j):
+                serials.append(ser)
+                first.append(fi)
+                lens.append(len(ser))
+            run += int(parts[i].sets[j]["count"])
+        off = np.zeros(len(lens) + 1, np.uint64)
+        off[1:] = np.cumsum(lens, dtype=np.uint64)
+        return SetExport(max([p.next_index for p in parts] or [0]), sets, np.frombuffer(b"".join(serials), np.uint8).copy(), off,
+                         np.array(first, np.uint64))
+
 
 def _attach_pem(o: "capi.Out", res: BatchResult, n: int, der_bytes: int):
     """Room for the PEM of every certificate of the batch (the worst case: all new)."""
@@ -91,6 +152,8 @@ class RawBatchResult:
 
 class GpuCertDatabase:
     """One ctmr_ctx = one GPU's share of the known-certificate state."""
+
+    _SETS = "ctmr_"   # prefix of the set read-back entry points this handle takes
 
     def __init__(self, device: int = 0, table_capacity: int = 1 << 22, issuer_cn_filter: bytes | str = b"",
                  log_expired_entries: bool = False, flags: int = 0, max_issuers: int = 0, max_batch_entries: int = 0,
@@ -341,6 +404,55 @@ class GpuCertDatabase:
         self._check(self._lib.ctmr_table_stats(self._h, C.byref(used), C.byref(cap)))
         return used.value, cap.value
 
+    # ------------------------------------------------------------------ the sets read back (list, members, export / import)
+    def _sets_fn(self, name):
+        return getattr(self._lib, self._SETS + name)
+
+    def list_sets(self, min_exp_hour: int | None = None, max_exp_hour: int | None = None) -> np.ndarray:
+        """Live sets with min_exp_hour <= exp_hour <= max_exp_hour (None = unbounded), canonical order, as a
+        capi.SET_INFO_DTYPE array (issuer_digest, exp_hour, count, member_off).  On a group member: that shard's sets."""
+        lo = -(1 << 63) if min_exp_hour is None else int(min_exp_hour)
+        hi = (1 << 63) - 1 if max_exp_hour is None else int(max_exp_hour)
+        fn, n = self._sets_fn("list_sets"), C.c_uint64(0)
+        self._check(fn(self._h, lo, hi, None, 0, C.byref(n)))
+        out = np.zeros(max(n.value, 1), capi.SET_INFO_DTYPE)
+        self._check(fn(self._h, lo, hi, capi.ptr(out), out.size, C.byref(n)))
+        return out[:n.value]
+
+    def set_members(self, exp_hour: int, issuer_digest: bytes):
+        """(serials in first-seen order, their first indices) of one set."""
+        fn, n = self._sets_fn("set_members"), C.c_uint64(0)
+        d = (C.c_uint8 * 32).from_buffer_copy(bytes(issuer_digest))
+        self._check(fn(self._h, int(exp_hour), d, None, 0, None, None, 0, C.byref(n)))
+        cap = max(n.value, 1)
+        blob, off, first = np.zeros(cap * capi.MAX_SERIAL, np.uint8), np.zeros(cap + 1, np.uint64), np.zeros(cap, np.uint64)
+        self._check(fn(self._h, int(exp_hour), d, capi.ptr(blob), blob.size, capi.ptr(off), capi.ptr(first), cap, C.byref(n)))
+        k = n.value
+        return [blob[int(off[i]):int(off[i + 1])].tobytes() for i in range(k)], first[:k].copy()
+
+    def export_sets(self) -> SetExport:
+        """Canonical export of every live set (include/ctmr.h): portable to a ctx or group of any size."""
+        fn, x = self._sets_fn("export_sets"), capi.SetExport()
+        self._check(fn(self._h, C.byref(x)))
+        sets = np.zeros(max(x.n_sets, 1), capi.SET_INFO_DTYPE)
+        serials = np.zeros(max(x.serial_bytes, 1), np.uint8)
+        off, first = np.zeros(x.n_members + 1, np.uint64), np.zeros(max(x.n_members, 1), np.uint64)
+        x.sets, x.sets_cap = capi.ptr(sets), sets.size
+        x.serials, x.serials_cap = capi.ptr(serials), serials.size
+        x.serial_off, x.first_index, x.members_cap = capi.ptr(off), capi.ptr(first), x.n_members
+        self._check(fn(self._h, C.byref(x)))
+        return SetExport(int(x.next_index), sets[:x.n_sets], serials[:x.serial_bytes], off[:x.n_members + 1], first[:x.n_members])
+
+    def import_sets(self, export: SetExport):
+        """Load an export into this EMPTY ctx / group (CtmrError otherwise); members keep their first indices."""
+        sets = np.ascontiguousarray(export.sets, capi.SET_INFO_DTYPE)
+        serials = np.ascontiguousarray(export.serials, np.uint8)
+        off, first = np.ascontiguousarray(export.serial_off, np.uint64), np.ascontiguousarray(export.first_index, np.uint64)
+        keep = [np.zeros(1, np.uint8) if a.size == 0 else a for a in (sets, serials, first)]
+        x = capi.SetExport(int(export.next_index), sets.size, first.size, serials.size, capi.ptr(keep[0]), sets.size,
+                           capi.ptr(keep[1]), serials.size, capi.ptr(off), capi.ptr(keep[2]), first.size)
+        self._check(self._sets_fn("import_sets")(self._h, C.byref(x)))
+
 
 class GpuCertGroup(GpuCertDatabase):
     """Several GPUs of one box behind ONE handle (ctmr_group_*): what the Go host calls in place of the worker pool of
@@ -366,6 +478,7 @@ class GpuCertGroup(GpuCertDatabase):
         if rc != 0:
             raise CtmrError(rc, (self._lib.ctmr_group_last_error(None) or b"").decode())
         self._h, self._owned = h, True
+        self._SETS = "ctmr_group_"
         self.devices, self.device, self.flags = list(devices), devices[0], flags
         self.members = [GpuCertDatabase(device=devices[r], flags=flags, _adopt=C.c_void_p(self._lib.ctmr_group_member(h, r)))
                         for r in range(len(devices))]
@@ -430,6 +543,9 @@ class GpuCertGroup(GpuCertDatabase):
                 d = (C.c_uint8 * 32).from_buffer_copy(bytes(issuer_digest))
                 grp._check(grp._lib.ctmr_group_set_cardinality(grp._h, int(exp_hour), d, C.byref(out)))
                 return out.value
+
+            def known(self_inner) -> list:
+                return grp.set_members(exp_hour, issuer_digest)[0]
         return _View()
 
     def issuer_counts(self) -> dict:

@@ -628,7 +628,132 @@ class GpuCertDatabase {
         return "";
     }
 
+    // ---- the sets read back out of the device (include/ctmr.h, "the sets read back")
+    struct DeviceSet {
+        ExpDate expDate;
+        Issuer issuer;
+        uint8_t digest[32];
+        uint64_t count;  // SetCardinality
+    };
+    // GetIssuerAndDatesFromCache (filesystemdatabase.go:59-100) + Count() per set, answered from HBM instead of a
+    // KEYS serials::* scan; [min_hour, max_hour] is ListExpirationDates(notBefore)'s range.  Canonical order.
+    std::pair<std::vector<DeviceSet>, Error> GetIssuerAndDatesFromDevice(int64_t min_hour = INT64_MIN, int64_t max_hour = INT64_MAX) {
+        std::vector<DeviceSet> out;
+        uint64_t n = 0;
+        int rc = group_ ? ctmr_group_list_sets(group_, min_hour, max_hour, nullptr, 0, &n) : ctmr_list_sets(ctx_, min_hour, max_hour, nullptr, 0, &n);
+        std::vector<ctmr_set_info> raw(n);
+        if (rc == CTMR_OK && n)
+            rc = group_ ? ctmr_group_list_sets(group_, min_hour, max_hour, raw.data(), n, &n) : ctmr_list_sets(ctx_, min_hour, max_hour, raw.data(), n, &n);
+        if (rc != CTMR_OK) return {out, lastError("ctmr_list_sets")};
+        for (uint64_t j = 0; j < n; ++j) {
+            DeviceSet d{ExpDate{raw[j].exp_hour}, Issuer::FromDigest(raw[j].issuer_digest), {}, raw[j].count};
+            std::memcpy(d.digest, raw[j].issuer_digest, 32);
+            out.push_back(d);
+        }
+        return {out, ""};
+    }
+
+    // KnownCertificates.Known() (knowncertificates.go:65-96) of one set, from HBM: its serials in first-seen order
+    std::pair<std::vector<Serial>, Error> KnownFromDevice(const ExpDate& expDate, const uint8_t issuer_digest[32]) {
+        std::vector<Serial> out;
+        uint64_t n = 0;
+        auto call = [&](uint8_t* ser, uint64_t ser_cap, uint64_t* off, uint64_t* first, uint64_t cap) {
+            return group_ ? ctmr_group_set_members(group_, expDate.hour, issuer_digest, ser, ser_cap, off, first, cap, &n)
+                          : ctmr_set_members(ctx_, expDate.hour, issuer_digest, ser, ser_cap, off, first, cap, &n);
+        };
+        int rc = call(nullptr, 0, nullptr, nullptr, 0);
+        if (rc != CTMR_OK) return {out, lastError("ctmr_set_members")};
+        if (!n) return {out, ""};
+        std::vector<uint8_t> blob(n * CTMR_MAX_SERIAL);
+        std::vector<uint64_t> off(n + 1), first(n);
+        rc = call(blob.data(), blob.size(), off.data(), first.data(), n);
+        if (rc != CTMR_OK) return {out, lastError("ctmr_set_members")};
+        for (uint64_t k = 0; k < n; ++k) out.push_back(Serial::FromBytes(blob.data() + off[k], off[k + 1] - off[k]));
+        return {out, ""};
+    }
+    std::pair<std::vector<Serial>, Error> KnownFromDevice(const ExpDate& expDate, const Issuer& issuer) {
+        uint8_t d[32];
+        if (!Base64URLDecode32(issuer.ID(), d)) return {{}, "KnownFromDevice: issuer id is not a base64url SHA-256 digest"};
+        return KnownFromDevice(expDate, d);
+    }
+
+    // A lost or never-written Redis rebuilt from the device: one SetInsert per member of every live set and one
+    // ExpireAt(expDate) per set (knowncertificates.go:44-47), in canonical order.  A cache with the pipelined
+    // extension gets all of them in one SetInsertBatch and one ExpireAtBatch.  The IssuerMetadata string sets
+    // ("issuer::" / "crl::") are process memory of the device path and are not part of the export.
+    Error RebuildRemoteCache(RemoteCache* target) {
+        ctmr_set_export x{};
+        int rc = exportSets(&x);  // NULL arrays: the sizes
+        if (rc != CTMR_OK) return lastError("ctmr_export_sets");
+        std::vector<ctmr_set_info> sets(x.n_sets + 1);
+        std::vector<uint8_t> serials(x.serial_bytes + 1);
+        std::vector<uint64_t> off(x.n_members + 1), first(x.n_members + 1);
+        x.sets = sets.data(); x.sets_cap = x.n_sets;
+        x.serials = serials.data(); x.serials_cap = x.serial_bytes;
+        x.serial_off = off.data(); x.first_index = first.data(); x.members_cap = x.n_members;
+        rc = exportSets(&x);
+        if (rc != CTMR_OK) return lastError("ctmr_export_sets");
+        BatchRemoteCache* pipelined = dynamic_cast<BatchRemoteCache*>(target);
+        std::vector<BatchRemoteCache::Insert> inserts;
+        std::vector<BatchRemoteCache::Expire> expires;
+        for (uint64_t j = 0; j < x.n_sets; ++j) {
+            const ExpDate e{sets[j].exp_hour};
+            KnownCertificates kc(e, Issuer::FromDigest(sets[j].issuer_digest), target);
+            const std::string key = kc.serialId();
+            for (uint64_t k = sets[j].member_off; k < sets[j].member_off + sets[j].count; ++k) {
+                std::string member(reinterpret_cast<const char*>(serials.data() + off[k]), (size_t)(off[k + 1] - off[k]));
+                if (pipelined) {
+                    inserts.push_back({key, std::move(member)});
+                } else {
+                    Error err = target->SetInsert(key, member).second;
+                    if (!ok(err)) return err;
+                }
+            }
+            if (pipelined) {
+                expires.push_back({key, e.ExpireTimeUnix()});
+            } else {
+                Error err = target->ExpireAt(key, e.ExpireTimeUnix());
+                if (!ok(err)) return err;
+            }
+        }
+        if (pipelined && !inserts.empty()) {
+            Error err = pipelined->SetInsertBatch(inserts).second;
+            if (!ok(err)) return err;
+        }
+        if (pipelined && !expires.empty()) return pipelined->ExpireAtBatch(expires);
+        return "";
+    }
+
   private:
+    int exportSets(ctmr_set_export* x) { return group_ ? ctmr_group_export_sets(group_, x) : ctmr_export_sets(ctx_, x); }
+    Error lastError(const char* what) const {
+        return std::string(what) + ": " + (group_ ? ctmr_group_last_error(group_) : ctmr_last_error(ctx_));
+    }
+    // Issuer.ID() back to its digest: base64.URLEncoding of 32 bytes (44 characters, one '=')
+    static bool Base64URLDecode32(const std::string& id, uint8_t out[32]) {
+        if (id.size() != 44) return false;
+        uint32_t acc = 0;
+        int bits = 0, n = 0;
+        for (char c : id) {
+            int v;
+            if (c >= 'A' && c <= 'Z') v = c - 'A';
+            else if (c >= 'a' && c <= 'z') v = c - 'a' + 26;
+            else if (c >= '0' && c <= '9') v = c - '0' + 52;
+            else if (c == '-') v = 62;
+            else if (c == '_') v = 63;
+            else if (c == '=') break;
+            else return false;
+            acc = (acc << 6) | (uint32_t)v;
+            bits += 6;
+            if (bits >= 8) {
+                bits -= 8;
+                if (n == 32) return false;
+                out[n++] = (uint8_t)(acc >> bits);
+            }
+        }
+        return n == 32;
+    }
+
     ctmr_ctx* ctx_;
     ctmr_group* group_ = nullptr;
     RemoteCache* cache_;

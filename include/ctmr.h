@@ -190,6 +190,62 @@ int ctmr_snapshot_size(ctmr_ctx* ctx, uint64_t* bytes);
 int ctmr_snapshot_save(ctmr_ctx* ctx, uint8_t* buf, uint64_t cap, uint64_t* written);
 int ctmr_snapshot_load(ctmr_ctx* ctx, const uint8_t* buf, uint64_t bytes);
 
+/* ---- the sets read back: list, members, canonical export / import ---------------------------- */
+/* What the reference reads out of Redis: KnownCertificates.Known() (storage/knowncertificates.go:65-96),
+ * GetIssuerAndDatesFromCache (storage/filesystemdatabase.go:59-100, a KEYS serials::* scan) and the walk of
+ * cmd/storage-statistics.  Semantics:
+ *   - a LIVE set is an (issuer, expDate) whose cardinality is > 0.  Sets emptied by ctmr_evict_expired keep their
+ *     first-seen memo on the device but no longer exist in Redis, so they are not listed.
+ *   - a MEMBER is a serial in the known-certificate table together with its first-seen global entry index.  Serials
+ *     longer than CTMR_MAX_SERIAL never entered the table (CTMR_ST_SERIAL_TOO_LONG), so they never appear.
+ *   - CANONICAL ORDER: sets by (issuer digest bytes, exp_hour) ascending, members of a set by first index ascending.
+ *     The order depends on the logical state only: a single ctx, a group of any size and the merge of the shards of a
+ *     peer group export byte-identical results for the same entries (entry i of a batch keeps global index
+ *     next_index + i in every shape).
+ *   - an export carries the Redis state (sets, members, cardinalities) and next_index.  It does NOT carry process
+ *     memory: the IssuerMetadata string memos (first_issuer_dn / first_crldp) and the first-seen memo of evicted sets.
+ *     An imported state therefore behaves like a restarted reference process against the same Redis.
+ * Buffers are HOST memory.  A call whose output pointers are NULL only reports the sizes (one (issuer, hour) table
+ * scan, plus one counting pass over the known-certificate table for the serial bytes of an export); buffers too small
+ * for the result give CTMR_E_BATCH_TOO_LARGE with the sizes reported all the same.
+ * On a member of a group (ctmr_group_member, or one rank of a ctmr_peer_* group) list, members and export cover the
+ * sets THAT shard owns; they are not collective, and merging the shards' exports in canonical order gives the group's. */
+typedef struct ctmr_set_info {
+    uint8_t issuer_digest[32];
+    int64_t exp_hour;
+    uint64_t count;       /* SetCardinality */
+    uint64_t member_off;  /* index of the set's first member in the member arrays (= running sum of the counts) */
+} ctmr_set_info;
+
+typedef struct ctmr_set_export {
+    uint64_t next_index;    /* out on export, in on import: the ctx's (group's) next global entry index (what the host-buffer
+                             * calls and preloads have used; callers of the device entry points choose the indices themselves) */
+    uint64_t n_sets, n_members, serial_bytes;  /* out on export (also for too-small / NULL buffers), in on import */
+    ctmr_set_info* sets;    /* [sets_cap] */
+    uint64_t sets_cap;
+    uint8_t* serials;       /* [serials_cap]: member k = serials[serial_off[k] .. serial_off[k+1]) */
+    uint64_t serials_cap;
+    uint64_t* serial_off;   /* [members_cap + 1] */
+    uint64_t* first_index;  /* [members_cap] */
+    uint64_t members_cap;
+} ctmr_set_export;
+
+/* GetIssuerAndDatesFromCache + Count(): the live sets with min_exp_hour <= exp_hour <= max_exp_hour (ListExpirationDates'
+ * notBefore is the lower bound), canonical order.  *n = number of sets. */
+int ctmr_list_sets(ctmr_ctx* ctx, int64_t min_exp_hour, int64_t max_exp_hour, ctmr_set_info* out, uint64_t cap, uint64_t* n);
+/* KnownCertificates.Known() of one set, members by first index; *n = number of members, serial_off [cap + 1].
+ * serials_cap >= CTMR_MAX_SERIAL * n always suffices. */
+int ctmr_set_members(ctmr_ctx* ctx, int64_t exp_hour, const uint8_t issuer_digest[32], uint8_t* serials, uint64_t serials_cap,
+                     uint64_t* serial_off, uint64_t* first_index, uint64_t cap, uint64_t* n);
+int ctmr_export_sets(ctmr_ctx* ctx, ctmr_set_export* x);
+/* Into an EMPTY ctx only (next_index == 0, no key in the table; else CTMR_E_INVALID), of any capacity: every member keeps
+ * its exported first index, next_index becomes the exported one, cardinalities and per-issuer counts follow from the
+ * keys, unknown issuer digests are registered (dense indices may differ from the source's; the canonical form does not
+ * show them).  Serials empty or longer than CTMR_MAX_SERIAL are CTMR_E_INVALID.  A rank of a ctmr_peer_* group loads
+ * the sets it owns only, so every rank can be handed the same full export; a member of an in-process group refuses:
+ * use ctmr_group_import_sets. */
+int ctmr_import_sets(ctmr_ctx* ctx, const ctmr_set_export* x);
+
 /* ---- device-resident entry points ---------------------------------------------------------- */
 /* Same path with every buffer already in HBM on ctx's device (benchmarks, multi-GPU orchestration,
  * hosts that receive entries by GPUDirect).  `stream` is a cudaStream_t passed as void*; NULL =
@@ -294,6 +350,14 @@ int ctmr_group_reset(ctmr_group* g);
 int ctmr_group_snapshot_size(ctmr_group* g, uint64_t* bytes);
 int ctmr_group_snapshot_save(ctmr_group* g, uint8_t* buf, uint64_t cap, uint64_t* written);
 int ctmr_group_snapshot_load(ctmr_group* g, const uint8_t* buf, uint64_t bytes);
+/* the sets of the whole group (every member scans its own shard on a thread of its own, the host merges the sorted
+ * lists); same outputs as the single-ctx calls, byte-identical to a single ctx over the same entries.  Import routes
+ * every set to its owner in THIS group, so an export moves between groups of any size and single ctxs. */
+int ctmr_group_list_sets(ctmr_group* g, int64_t min_exp_hour, int64_t max_exp_hour, ctmr_set_info* out, uint64_t cap, uint64_t* n);
+int ctmr_group_set_members(ctmr_group* g, int64_t exp_hour, const uint8_t issuer_digest[32], uint8_t* serials, uint64_t serials_cap,
+                           uint64_t* serial_off, uint64_t* first_index, uint64_t cap, uint64_t* n);
+int ctmr_group_export_sets(ctmr_group* g, ctmr_set_export* x);
+int ctmr_group_import_sets(ctmr_group* g, const ctmr_set_export* x);
 
 /* ---- several GPUs, one PROCESS PER GPU (torchrun-style launches; SURVEY.md §8(e)) ------------------------------ */
 /* Every rank creates its ctx with the same capacities, exports a handle, gathers all handles by whatever means the
